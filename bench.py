@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config C]            # our CUDA path
   python bench.py --impl reference --steps K --warmup W [--config C]    # reference libzstd on the host cores
+  python bench.py ... --dump-outputs DIR                                # also write the last timed step's frames to DIR
 
 --config selects one of BASELINE.json's workloads (default 2, the one the metric is quoted on):
   2  datagen -g1GB -P50, level 1, one frame per GPU (weak scaling: every rank owns one 1 GiB shard, seed = rank)
@@ -340,6 +341,24 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------------------------- our arm
+DUMP_SAMPLES = 4 << 20          # compressed bytes kept by --dump-outputs: 16 MiB as float32 + 32 MiB of float64 positions
+
+
+def dump_outputs(dirname, frames: bytes, frame_sizes):
+    """What the timed path returned in its last step, as .npy files that two builds can be compared by: the compressed
+    size of every frame, and the compressed bytes (all of them, or a fixed seeded sample of DUMP_SAMPLES positions
+    with those positions alongside)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    b = np.frombuffer(frames, dtype=np.uint8)
+    if b.size > DUMP_SAMPLES:
+        pos = np.sort(np.random.default_rng(0).integers(0, b.size, DUMP_SAMPLES))
+        np.save(os.path.join(dirname, "compressed_sample_positions.npy"), pos.astype(np.float64))
+        b = b[pos]
+    np.save(os.path.join(dirname, "compressed_bytes.npy"), b.astype(np.float32))
+    np.save(os.path.join(dirname, "frame_sizes.npy"), np.asarray(frame_sizes, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -500,6 +519,8 @@ def run_ours(args):
 
     # ---- parity of what was timed (outside the timed region) ----
     assert bytes(h_dst[:ce].numpy()) == got_dev, "host-path and device-path frames differ"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, got_dev, frame_sizes)
     digest = hashlib.sha256(wl.src).hexdigest()
     digests = [digest]
     if world > 1:
@@ -591,6 +612,7 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the workload (development only; 1.0 = the BASELINE size)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-decode", action="store_true", help="skip the GPU decompression round trip (configs 2 and 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy (rank 0)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

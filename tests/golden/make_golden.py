@@ -29,10 +29,10 @@ def main():
             case = make_seqstore(rng)
             if case is None:
                 continue
-            r1, b1, r2, b2 = run_both(case)
-            assert (r1, b1) == (r2, b2)
+            r1, h1, r2, b2 = run_both(case)
+            assert (r1, h1) == (r2, zref.sha16(b2))
             if 0 < r1 < (1 << 60) and len(vectors) < 40 and draw % 3 == 0:
-                vectors.append({"seed": seed, "draw": draw, "size": r1, "sha256": zref.sha(b1)})
+                vectors.append({"seed": seed, "draw": draw, "size": r1, "sha256": zref.sha(b2)})
     json.dump(vectors, open(os.path.join(HERE, "entropy_vectors.json"), "w"), indent=1)
 
     os.makedirs(os.path.join(HERE, "inputs"), exist_ok=True)

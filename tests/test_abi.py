@@ -41,12 +41,10 @@ def test_helpers_match_reference_semantics():
     assert L.ZSTD_isError(L.ZSTD_compressBound(0xFF00FF00FF00FF00))      # srcSize_wrong
     assert L.ZSTD_getErrorCode(L.ZSTD_compressBound(0xFF00FF00FF00FF00)) == 72
     assert not L.ZSTD_isError(12345)
-    if zref.have_ref():
-        R = zref.ref()
-        for code in (0, 1, 10, 30, 32, 40, 42, 44, 46, 60, 62, 64, 66, 70, 72, 74, 119):
-            v = (1 << 64) - code if code else 0
-            assert L.ZSTD_getErrorName(v) == R.ZSTD_getErrorName(v), code
-            assert bool(L.ZSTD_isError(v)) == bool(R.ZSTD_isError(v))
+    for code in (0, 1, 10, 30, 32, 40, 42, 44, 46, 60, 62, 64, 66, 70, 72, 74, 119):
+        v = (1 << 64) - code if code else 0
+        assert L.ZSTD_getErrorName(v).decode() == zref.ref_error_name(v), code
+        assert bool(L.ZSTD_isError(v)) == bool(zref.ref_call("ZSTD_isError", v))
 
 
 def test_context_lifecycle_without_gpu():
@@ -91,29 +89,6 @@ def test_header_is_valid_c99_and_links(tmp_path):
     subprocess.check_call(cmd)
     out = subprocess.check_output([str(exe)], text=True)
     assert out.split()[0] == "10506" and "too small" in out
-
-
-REF_EXAMPLES = "/root/reference/examples"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_EXAMPLES), reason="reference tree absent (GPU box)")
-@pytest.mark.parametrize("example", ["simple_compression.c", "multiple_simple_compression.c", "dictionary_compression.c"])
-def test_reference_examples_compile_and_link_unmodified(tmp_path, example):
-    """The reference's own example programs (examples/simple_compression.c:28 ZSTD_compress, multiple_simple_compression.c:74
-    ZSTD_compressCCtx, dictionary_compression.c ZSTD_createCDict / ZSTD_compress_usingCDict), compiled UNMODIFIED against the
-    STOCK lib/zstd.h, link against this library alone: every compression symbol they use is exported with the reference's
-    signature.  (Compile + link only: running them needs a GPU.)"""
-    import shutil, subprocess
-    gcc = shutil.which("gcc")
-    if not gcc:
-        pytest.skip("no gcc")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    libdir = os.path.join(root, "zstd_b200")
-    exe = tmp_path / "example"
-    cmd = [gcc, "-O1", "-I", "/root/reference/lib", "-I", REF_EXAMPLES, os.path.join(REF_EXAMPLES, example), "-o", str(exe),
-           "-L", libdir, "-lzstd_b200", "-Wl,-rpath," + libdir, "-L/usr/local/cuda/lib64", "-Wl,-rpath,/usr/local/cuda/lib64"]
-    subprocess.check_call(cmd)
-    assert os.path.exists(exe)
 
 
 def test_soname_build_target(tmp_path):

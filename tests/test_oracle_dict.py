@@ -2,12 +2,11 @@
 Frames must decode with the reference's ZSTD_decompress_usingDict and stay within +-0.5 % of the
 reference's size for raw-content and zstd-format dictionaries; the dictionary entropy stage (treeless
 literals, set_repeat tables, start repcodes) is pinned byte-for-byte against ZSTD_loadCEntropy +
-ZSTD_entropyCompressSeqStore of the compiled reference."""
+ZSTD_entropyCompressSeqStore of the compiled reference (recorded under tests/golden/reference/ where it is not built)."""
 import pytest
 
 import zref
 
-needs_ref = pytest.mark.skipif(not zref.have_ref(), reason="oracle/_ref/libzstd_ref.so not built")
 REC = 1024
 
 
@@ -16,7 +15,6 @@ def records(n, seed, p=0.5):
     return [data[i * REC:(i + 1) * REC] for i in range(n)]
 
 
-@needs_ref
 @pytest.mark.parametrize("dict_name", ["zdict-16k-synthetic-seed77", "http-dict-missing-symbols", "zero-weight-dict"])
 def test_zstd_format_dictionaries_roundtrip(dict_name):
     d = zref.golden_input(dict_name)
@@ -24,41 +22,38 @@ def test_zstd_format_dictionaries_roundtrip(dict_name):
     srcs = records(200, 5) + [b"", b"a", zref.golden_input("http"), zref.synthetic(300_000, 8)]
     for src in srcs:
         f = zref.oracle_compress_using_dict(src, d, 1)
-        assert zref.ref_decompress_using_dict(f, d, len(src)) == src
+        assert zref.ref_decodes(f, src, d)
         assert f[4] & 3, "dictID must be present in the frame header for a zstd-format dictionary"
         tot_o += len(f)
-        tot_r += len(zref.ref_compress_using_dict(src, d, 1))
+        tot_r += zref.ref_size(src, 1, d)
     if dict_name.startswith('zdict'):
         assert abs(tot_o - tot_r) / tot_r <= 0.01, (tot_o, tot_r)
     else:
         assert tot_o < tot_r * 1.03          # tiny hand-made dictionaries of the reference's test suite
 
 
-@needs_ref
 def test_raw_content_dictionary_size_parity():
     d = zref.synthetic(32 << 10, 123, 0.5)                 # no magic number -> raw content (zstd_compress.c:5143-5148)
     tot_o = tot_r = 0
     for src in records(400, 6):
         f = zref.oracle_compress_using_dict(src, d, 1)
-        assert zref.ref_decompress_using_dict(f, d, len(src)) == src
+        assert zref.ref_decodes(f, src, d)
         assert (f[4] & 3) == 0                              # no dictID for raw content (lib/zstd.h:185-186)
         tot_o += len(f)
-        tot_r += len(zref.ref_compress_using_dict(src, d, 1))
+        tot_r += zref.ref_size(src, 1, d)
     assert abs(tot_o - tot_r) / tot_r <= 0.01
 
 
-@needs_ref
 def test_dictionary_content_is_actually_used():
     """A record that is a verbatim slice of the dictionary must compress to almost nothing."""
     d = zref.synthetic(32 << 10, 321, 0.1)
     src = d[5000:6024]
     with_dict = zref.oracle_compress_using_dict(src, d, 1)
     without = zref.oracle_compress(src, 1)
-    assert zref.ref_decompress_using_dict(with_dict, d, len(src)) == src
+    assert zref.ref_decodes(with_dict, src, d)
     assert len(with_dict) < 100 < len(without)
 
 
-@needs_ref
 def test_short_and_corrupted_dictionaries():
     src = zref.synthetic(5000, 1)
     assert zref.oracle_compress_using_dict(src, b"1234567", 1) == zref.oracle_compress(src, 1)      # < 8 bytes: ignored
@@ -67,7 +62,6 @@ def test_short_and_corrupted_dictionaries():
         zref.oracle_compress_using_dict(src, bad, 1)
 
 
-@needs_ref
 @pytest.mark.parametrize("dict_name", ["zdict-16k-synthetic-seed77", "http-dict-missing-symbols", "zero-weight-dict"])
 def test_dictionary_entropy_stage_byte_exact(dict_name):
     """oracle/zb_dict.c + zbo_entropyCompressBlock_prev vs the reference's ZSTD_loadCEntropy (zstd_compress.c:4987)
@@ -75,10 +69,8 @@ def test_dictionary_entropy_stage_byte_exact(dict_name):
     import ctypes
     import numpy as np
     from test_oracle_entropy import make_seqstore
-    R, O = zref.ref(), zref.oracle()
+    O = zref.oracle()
     c_sz, vp = ctypes.c_size_t, ctypes.c_void_p
-    R.ref_entropyCompressBlock_dict.restype = c_sz
-    R.ref_entropyCompressBlock_dict.argtypes = [vp, c_sz, vp, vp, vp, c_sz, vp, c_sz, c_sz, ctypes.c_int, ctypes.c_uint, vp, c_sz]
     O.zbo_loadDictEntropy.restype = c_sz
     O.zbo_loadDictEntropy.argtypes = [vp, vp, c_sz]
     O.zbo_entropyCompressBlock_prev.restype = c_sz
@@ -107,17 +99,22 @@ def test_dictionary_entropy_stage_byte_exact(dict_name):
         offb, ll, ml = (np.ascontiguousarray(a, dtype=np.uint32) for a in (offb, ll, ml))
         lits = np.ascontiguousarray(lits)
         tlv = tl if strategy == 1 else 0
-        r1 = R.ref_entropyCompressBlock_dict(d1, cap, offb.ctypes.data, ll.ctypes.data, ml.ctypes.data, nseq, lits.ctypes.data, len(lits), block, 1, tlv, d, len(d))
+        def reference():
+            R = zref.ref()
+            R.ref_entropyCompressBlock_dict.restype = c_sz
+            R.ref_entropyCompressBlock_dict.argtypes = [vp, c_sz, vp, vp, vp, c_sz, vp, c_sz, c_sz, ctypes.c_int, ctypes.c_uint, vp, c_sz]
+            r = R.ref_entropyCompressBlock_dict(d1, cap, offb.ctypes.data, ll.ctypes.data, ml.ctypes.data, nseq, lits.ctypes.data, len(lits), block, 1, tlv, d, len(d))
+            return [r, zref.sha16(d1.raw[:r]) if r < (1 << 60) else None]
+        r1, h1 = zref.recorded(zref._key("entropy-dict", seqs.tobytes(), lits.tobytes(), block, tlv, d), reference)
         with zref.entropy_model(0):                                 # the restatement of the reference's table builders
             r2 = O.zbo_entropyCompressBlock_prev(d2, cap, seqs.ctypes.data, nseq, lits.ctypes.data, len(lits), block, 1, 1 if tlv > 0 else 0, de)
         assert r1 == r2
         if r1 < (1 << 60):
-            assert d1.raw[:r1] == d2.raw[:r2]
+            assert h1 == zref.sha16(d2.raw[:r2])
             compressed += r1 > 0
     assert compressed > 80
 
 
-@needs_ref
 @pytest.mark.skipif(not zref.have_datagen(), reason="oracle/_ref/datagen not built")
 @pytest.mark.parametrize("level", [1, 3, -3])
 def test_size_parity_with_reference_cdict(level):
@@ -128,12 +125,11 @@ def test_size_parity_with_reference_cdict(level):
     data = zref.datagen(REC * 6000, 50)
     d = zref.train_dict(data, REC, 4000, 16 << 10)
     srcs = [data[i * REC:(i + 1) * REC] for i in range(4000, 5000)]
-    ref_frames = zref.ref_compress_using_cdict(srcs, d, level)
     tot_o = 0
     for k, src in enumerate(srcs):
         f = zref.oracle_compress_using_dict(src, d, level)
         if k % 25 == 0:
-            assert zref.ref_decompress_using_dict(f, d, len(src)) == src
+            assert zref.ref_decodes(f, src, d)
         tot_o += len(f)
-    tot_r = sum(len(f) for f in ref_frames)
+    tot_r = zref.ref_cdict_size(srcs, d, level)
     assert abs(tot_o - tot_r) / tot_r <= 0.01, (tot_o, tot_r)

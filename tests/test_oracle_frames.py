@@ -1,5 +1,6 @@
 """Oracle at frame level: every frame decodes with the reference decoder, sizes stay within the
-two-sided bound of zref.size_delta_ok on the BASELINE inputs, parameter derivation equals the reference's, golden fixtures."""
+two-sided bound of zref.size_delta_ok on the BASELINE inputs, parameter derivation equals the reference's, golden fixtures.
+The reference's answers come from the compiled library where it is built and from tests/golden/reference/ elsewhere."""
 import ctypes
 import json
 import os
@@ -8,10 +9,6 @@ import pytest
 
 import zref
 
-needs_ref = pytest.mark.skipif(not zref.have_ref(), reason="oracle/_ref/libzstd_ref.so not built")
-
-
-@needs_ref
 @pytest.mark.parametrize("level", [1, 2, 3, 4, 0, -1, -3, -7])
 @pytest.mark.parametrize("size", [0, 1, 100, 1000, 16 << 10, (16 << 10) + 1, 100_000, 128 << 10, (128 << 10) + 1,
                                   256 << 10, (256 << 10) + 1, 1 << 20, 5 << 20, 600 << 20])
@@ -23,19 +20,21 @@ def test_cparams_match_reference(level, size):
     O = zref.oracle()
     O.zbo_getCParams.restype = CP
     O.zbo_getCParams.argtypes = [ctypes.c_int, ctypes.c_ulonglong, ctypes.c_size_t]
-    out = (ctypes.c_uint * 7)()
-    zref.ref().ref_getCParams_simpleApi(level, size, 0, out)
+    def reference():
+        out = (ctypes.c_uint * 7)()
+        zref.ref().ref_getCParams_simpleApi(level, size, 0, out)
+        return list(out)
+    out = zref.recorded(zref._key("cparams", level, size), reference)
     ours = O.zbo_getCParams(level, size, 0)
     if out[6] > 2:
         pytest.skip("reference strategy above dfast: out of scope, served by the dfast row")
-    assert [ours.windowLog, ours.chainLog, ours.hashLog, ours.searchLog, ours.minMatch, ours.targetLength, ours.strategy] == list(out)
+    assert [ours.windowLog, ours.chainLog, ours.hashLog, ours.searchLog, ours.minMatch, ours.targetLength, ours.strategy] == out
 
 
-@needs_ref
 def test_compress_bound_matches_reference():
-    O, R = zref.oracle(), zref.ref()
+    O = zref.oracle()
     for n in [0, 1, 100, 1 << 10, 128 << 10, (128 << 10) - 1, (128 << 10) + 1, 1 << 20, 1 << 30, 5 << 30]:
-        assert O.zbo_compressBound(n) == R.ZSTD_compressBound(n)
+        assert O.zbo_compressBound(n) == zref.ref_call("ZSTD_compressBound", n)
 
 
 EDGE = {
@@ -52,19 +51,17 @@ for _n in (SEG - 1, SEG, SEG + 1, SEG + 6, SEG + 7, SEG + 8, 2 * SEG + 3, 8 * SE
 EDGE["seg-rep"] = (zref.synthetic(5000, 77, 0.3) * 30)[: 9 * SEG + 123]        # matches that want to run across every segment end
 
 
-@needs_ref
 @pytest.mark.parametrize("name", sorted(EDGE))
 @pytest.mark.parametrize("level", [1, -3, 3])
 def test_roundtrip_edge_cases(name, level):
     src = EDGE[name]
     frame = zref.oracle_compress(src, level)
-    assert zref.ref_decompress(frame, len(src)) == src
-    assert len(frame) <= zref.ref().ZSTD_compressBound(len(src))
-    assert zref.ref().ZSTD_getFrameContentSize(frame, len(frame)) == len(src)       # fuzzer.c:4565-4573
+    assert zref.ref_decodes(frame, src)
+    assert len(frame) <= zref.ref_call("ZSTD_compressBound", len(src))
+    assert zref.ref_frame_content_size(frame) == len(src)                           # fuzzer.c:4565-4573
     assert zref.oracle_compress(src, level) == frame                                  # determinism (fuzz/simple_round_trip.c)
 
 
-@needs_ref
 def test_dst_too_small_is_an_error_not_an_overflow():
     src = zref.synthetic(300_000, 1)
     full = zref.oracle_compress(src, 1)
@@ -98,12 +95,10 @@ def test_golden_frames_fixture():
         out = zref.oracle_compress(data, int(level))
         assert len(out) == rec["oracle_size"] and zref.sha(out) == rec["oracle_sha256"], key
         assert zref.size_delta_ok(len(out), rec["ref_size"], len(data), name.startswith("synthetic")), (key, len(out), rec["ref_size"])
-        if zref.have_ref():
-            assert zref.ref_decompress(out, len(data)) == data
-            assert len(zref.ref_compress(data, int(level))) == rec["ref_size"]
+        assert zref.ref_decodes(out, data)
+        assert zref.ref_size(data, int(level)) == rec["ref_size"]
 
 
-@needs_ref
 @pytest.mark.skipif(not zref.have_datagen(), reason="reference datagen binary not built")
 @pytest.mark.parametrize("p,level,size", [(50, 1, 16 << 20), (30, -3, 16 << 20), (90, 3, 64 << 20)])
 def test_size_close_to_reference(p, level, size):
@@ -111,13 +106,12 @@ def test_size_close_to_reference(p, level, size):
     inside the two-sided bound of zref.size_delta_ok (measured: -0.65 %, -0.3 %, -1.2 %)."""
     src = zref.datagen(size, p)
     ours = zref.oracle_compress(src, level)
-    ref = zref.ref_compress(src, level)
-    assert zref.ref_decompress(ours, len(src)) == src
-    delta = (len(ours) - len(ref)) / len(ref)
-    assert zref.size_delta_ok(len(ours), len(ref), len(src)), f"size delta {delta:+.4%} (ours {len(ours)}, reference {len(ref)})"
+    ref = zref.ref_size(src, level)
+    assert zref.ref_decodes(ours, src)
+    delta = (len(ours) - ref) / ref
+    assert zref.size_delta_ok(len(ours), ref, len(src)), f"size delta {delta:+.4%} (ours {len(ours)}, reference {ref})"
 
 
-@needs_ref
 @pytest.mark.skipif(not zref.have_datagen(), reason="reference datagen binary not built")
 @pytest.mark.parametrize("level", [1, 3, -3])
 @pytest.mark.parametrize("p", [30, 50, 90])
@@ -125,6 +119,6 @@ def test_one_rule_for_all_datagen_types(p, level):
     """the same table sizes and insertion rule serve P30, P50 and P90 (round 1 fitted level 3 to P90 alone): 8 MiB samples"""
     src = zref.datagen(8 << 20, p)
     ours = zref.oracle_compress(src, level)
-    ref = zref.ref_compress(src, level)
-    assert zref.ref_decompress(ours, len(src)) == src
-    assert zref.size_delta_ok(len(ours), len(ref), len(src)), f"{(len(ours) - len(ref)) / len(ref):+.4%}"
+    ref = zref.ref_size(src, level)
+    assert zref.ref_decodes(ours, src)
+    assert zref.size_delta_ok(len(ours), ref, len(src)), f"{(len(ours) - ref) / ref:+.4%}"

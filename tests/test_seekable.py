@@ -1,6 +1,7 @@
 """Seek table writer (SURVEY §8f rank 4), CPU only: frames come from the oracle, the table from the product's host code,
 and the reference's own seekable reader (contrib/seekable_format/zstdseek_decompress.c, compiled in place into
-oracle/_ref/libzstd_seekable_ref.so) must find every frame and decompress arbitrary ranges."""
+oracle/_ref/libzstd_seekable_ref.so; its answers are recorded under tests/golden/reference/ for machines without it) must
+find every frame and decompress arbitrary ranges."""
 import ctypes
 import os
 import random
@@ -11,10 +12,11 @@ import zref
 import zstd_b200
 
 SEEK_SO = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libzstd_seekable_ref.so")
-pytestmark = pytest.mark.skipif(not (zref.have_ref() and os.path.exists(SEEK_SO)), reason="reference seekable reader not built")
 
 
-def test_reference_reader_accepts_our_seek_table():
+def _seekable_reader(blob, ranges):
+    """what the reference's seekable reader reports for blob: the number of frames, each frame's compressed offset and
+    a digest (zref.sha16) of each decompressed range (start, length)"""
     S = ctypes.CDLL(SEEK_SO)
     S.ZSTD_seekable_create.restype = ctypes.c_void_p
     S.ZSTD_seekable_initBuff.restype = ctypes.c_size_t
@@ -26,6 +28,21 @@ def test_reference_reader_accepts_our_seek_table():
     S.ZSTD_seekable_getFrameCompressedOffset.restype = ctypes.c_ulonglong
     S.ZSTD_seekable_getFrameCompressedOffset.argtypes = [ctypes.c_void_p, ctypes.c_uint]
     S.ZSTD_seekable_free.argtypes = [ctypes.c_void_p]
+    zs = S.ZSTD_seekable_create()
+    r = S.ZSTD_seekable_initBuff(zs, blob, len(blob))
+    assert not zref.ref().ZSTD_isError(r)
+    n = S.ZSTD_seekable_getNumFrames(zs)
+    offsets = [S.ZSTD_seekable_getFrameCompressedOffset(zs, i) for i in range(n)]
+    digests = []
+    for a, k in ranges:
+        out = ctypes.create_string_buffer(k)
+        got = S.ZSTD_seekable_decompress(zs, out, k, a)
+        digests.append(zref.sha16(out.raw) if got == k else None)
+    S.ZSTD_seekable_free(zs)
+    return [n, offsets, digests]
+
+
+def test_reference_reader_accepts_our_seek_table():
     rng = random.Random(5)
     sizes = [1024] * 20 + [0, 70_000, 300_000, 5, 128 << 10]
     src = zref.synthetic(sum(sizes), 9, 0.5)
@@ -35,21 +52,19 @@ def test_reference_reader_accepts_our_seek_table():
     blob = b"".join(frames) + zstd_b200.seek_table([len(f) for f in frames], sizes)
     assert len(blob) == sum(len(f) for f in frames) + 17 + 8 * len(sizes)
     assert blob[-4:] == bytes.fromhex("b1ea928f")                                   # Seekable_Magic_Number, little-endian
-    assert zref.ref_decompress(blob, len(src)) == src                               # the table is a skippable frame for a plain decoder
-    zs = S.ZSTD_seekable_create()
-    r = S.ZSTD_seekable_initBuff(zs, blob, len(blob))
-    assert not zref.ref().ZSTD_isError(r)
-    assert S.ZSTD_seekable_getNumFrames(zs) == len(sizes)
-    pos = 0
-    for i, f in enumerate(frames):
-        assert S.ZSTD_seekable_getFrameCompressedOffset(zs, i) == pos
-        pos += len(f)
+    assert zref.ref_decodes(blob, src)                                              # the table is a skippable frame for a plain decoder
+    ranges = []
     for _ in range(50):
         a = rng.randrange(0, len(src)); n = rng.randrange(1, min(100_000, len(src) - a) + 1)
-        out = ctypes.create_string_buffer(n)
-        got = S.ZSTD_seekable_decompress(zs, out, n, a)
-        assert got == n and out.raw == src[a:a + n], (a, n)
-    S.ZSTD_seekable_free(zs)
+        ranges.append((a, n))
+    nframes, offsets, digests = zref.recorded(zref._key("seekable", blob, ranges), lambda: _seekable_reader(blob, ranges))
+    assert nframes == len(sizes)
+    pos = 0
+    for i, f in enumerate(frames):
+        assert offsets[i] == pos
+        pos += len(f)
+    for (a, n), h in zip(ranges, digests):
+        assert h == zref.sha16(src[a:a + n]), (a, n)
 
 
 def test_seek_table_errors():

@@ -212,6 +212,143 @@ def golden_input(name: str) -> bytes:
         return f.read()
 
 
+# ----------------------------------------------------------------------------------------------- recorded reference results
+# The tests compare with the reference library (the original zstd, built into oracle/_ref/ by `make -C oracle ref` where
+# its source tree is at hand).  Where that library is absent, the same comparisons are answered from what it returned
+# before, stored in tests/golden/reference/results.json.xz: sizes, digests, small values, and the reference encoder's
+# frames that the decoder tests feed to this project's decoders, those of at most STORED_FRAME_MAX bytes (the larger ones
+# would make the repository heavy; a case that needs one is skipped where the library is absent).  A run with
+# ZB_RECORD_REFERENCE=1 and the library present adds every result it asks for to that file.
+RECORDED = os.path.join(GOLDEN, "reference")
+RECORD = os.environ.get("ZB_RECORD_REFERENCE") == "1"
+STORED_FRAME_MAX = 8 << 10
+_recorded = None
+_new_results = {}
+
+
+def sha16(b) -> str:
+    return hashlib.sha256(b).hexdigest()[:16]
+
+
+def _key(*parts) -> str:
+    return ":".join("-" if p is None else sha16(p) if isinstance(p, (bytes, bytearray)) else str(p) for p in parts)
+
+
+def _load_recorded():
+    global _recorded
+    if _recorded is None:
+        import json
+        import lzma
+        with lzma.open(os.path.join(RECORDED, "results.json.xz"), "rt") as f:
+            _recorded = json.load(f)
+    return _recorded
+
+
+def _missing(key):
+    return LookupError(f"no recorded reference result for {key}: record it with ZB_RECORD_REFERENCE=1 where oracle/_ref/ is built")
+
+
+def recorded(key: str, compute):
+    """compute() with the reference library where it is built, its recorded result elsewhere (JSON values)"""
+    if have_ref():
+        v = compute()
+        if RECORD:
+            _new_results[key] = v
+        return v
+    results = _load_recorded()
+    if key not in results:
+        raise _missing(key)
+    return results[key]
+
+
+def recorded_frame(key: str, compute) -> bytes:
+    """as recorded(), for frames: those longer than STORED_FRAME_MAX are not stored, and a test that asks for one where
+    the library is absent is skipped"""
+    import base64
+    if have_ref():
+        v = compute()
+        if RECORD and len(v) <= STORED_FRAME_MAX:
+            _new_results[key] = base64.b64encode(v).decode()
+        return v
+    results = _load_recorded()
+    if key not in results:
+        import pytest
+        pytest.skip(f"the reference's frame for this input is not stored in tests/golden/reference/ (at most {STORED_FRAME_MAX} bytes are)")
+    return base64.b64decode(results[key])
+
+
+def _save_recorded():
+    if not _new_results:
+        return
+    import fcntl
+    import json
+    import lzma
+    os.makedirs(RECORDED, exist_ok=True)
+    with open(os.path.join(RECORDED, ".lock"), "w") as lock:       # test workers of one run may finish together
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        path = os.path.join(RECORDED, "results.json.xz")
+        results = {}
+        if os.path.exists(path):
+            with lzma.open(path, "rt") as f:
+                results = json.load(f)
+        results.update(_new_results)
+        with lzma.open(path, "wt", preset=9) as f:
+            json.dump(results, f, separators=(",", ":"), sort_keys=True)
+    os.remove(os.path.join(RECORDED, ".lock"))
+
+
+if RECORD:
+    import atexit
+    atexit.register(_save_recorded)
+
+
+def ref_frame(src: bytes, level: int, dict_bytes: bytes = None) -> bytes:
+    """the reference encoder's frame of src (ZSTD_compress, or ZSTD_compress_usingDict with dict_bytes)"""
+    return recorded_frame(_key("frame", src, level, dict_bytes),
+                          lambda: ref_compress(src, level) if dict_bytes is None else ref_compress_using_dict(src, dict_bytes, level))
+
+
+def ref_size(src: bytes, level: int, dict_bytes: bytes = None) -> int:
+    """size of the reference encoder's frame of src"""
+    return recorded(_key("size", src, level, dict_bytes),
+                    lambda: len(ref_compress(src, level) if dict_bytes is None else ref_compress_using_dict(src, dict_bytes, level)))
+
+
+def ref_cdict_size(srcs, dict_bytes: bytes, level: int) -> int:
+    """summed size of the reference's ZSTD_compress_usingCDict frames of srcs"""
+    return recorded(_key("cdict-size", b"".join(sha16(s).encode() for s in srcs), dict_bytes, level),
+                    lambda: sum(len(f) for f in ref_compress_using_cdict(srcs, dict_bytes, level)))
+
+
+def ref_decoded_digest(frame: bytes, cap: int, dict_bytes: bytes = None):
+    """sha16 of what the reference decoder makes of frame (concatenated frames allowed), None where it reports an error"""
+    def run():
+        try:
+            out = ref_decompress(frame, cap) if dict_bytes is None else ref_decompress_using_dict(frame, dict_bytes, cap)
+        except ValueError:
+            return None
+        return sha16(out)
+    return recorded(_key("decode", frame, cap, dict_bytes), run)
+
+
+def ref_decodes(frame: bytes, src: bytes, dict_bytes: bytes = None) -> bool:
+    """the reference decoder turns frame back into src"""
+    return ref_decoded_digest(frame, len(src), dict_bytes) == sha16(src)
+
+
+def ref_call(name: str, *args):
+    """a function of the reference library that takes and returns integers (declared in ref())"""
+    return recorded(_key(name, *args), lambda: int(getattr(ref(), name)(*args)))
+
+
+def ref_error_name(code: int) -> str:
+    return recorded(_key("ZSTD_getErrorName", code), lambda: ref().ZSTD_getErrorName(code).decode())
+
+
+def ref_frame_content_size(frame: bytes) -> int:
+    return recorded(_key("ZSTD_getFrameContentSize", frame), lambda: int(ref().ZSTD_getFrameContentSize(frame, len(frame))))
+
+
 import contextlib
 
 
